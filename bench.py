@@ -2,6 +2,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # our arm (N>1: launched under torchrun)
     python bench.py --impl reference --gpus N --steps K ...   # CPU arm: the reference's path as ported by oracle/
+    python bench.py ... --dump-outputs DIR                    # + DIR/<name>.npy: what the last timed update step computed
 
 Workload (config.workload): the headline config ``configs[2]`` — Qwen2.5-7B (H=3584, V=152064) GRPO, math-shape
 synthetic rollouts, G=8, 2k context — weak-scaled: 16 prompts x 8 rollouts = 128 rows (~100k response tokens) per
@@ -36,6 +37,7 @@ import torch
 
 ROOT = Path(__file__).resolve().parent
 sys.path.insert(0, str(ROOT))
+sys.dont_write_bytecode = True  # the benchmark writes nothing into the tree it runs from (which may be read-only)
 # stdout carries exactly one JSON line (rank 0).  Libraries (NCCL's version banner, ...) write to fd 1 as well, so
 # fd 1 is pointed at stderr for the life of the process and the result goes to a private duplicate of the real stdout.
 _RESULT_OUT = os.fdopen(os.dup(1), "w")
@@ -102,8 +104,8 @@ _CPU_CACHE: dict = {}
 
 
 def _reference_host_stages(episodes, spec):
-    """C1-C3 of BASELINE.md section 4 on the reference's OWN code (unmodified, from /root/reference or the install under
-    baseline/_ref; third-party imports it cannot resolve here are stubbed by oracle/ref_harness): episodes -> groups ->
+    """C1-C3 of BASELINE.md section 4 on the reference's OWN code (unmodified, located by oracle/ref_harness, which also
+    stubs the third-party imports it cannot resolve here): episodes -> groups ->
     rejection filter -> numpy float64 advantages -> Python prefix-merge packing into the padded DataProto -> token-level
     advantage broadcast.  Returns (seconds, response tokens, rows as python lists for the loss sample, adv by uid)."""
     from types import SimpleNamespace
@@ -203,6 +205,35 @@ def cpu_reference_step(episodes, spec, loss_kw, sample_tokens: int, seed: int = 
 
 
 # --------------------------------------------------------------------------------------------------
+# --dump-outputs: what the timed path computed, for comparing two builds output by output
+# --------------------------------------------------------------------------------------------------
+DUMP_SAMPLE = 1 << 21  # elements kept of a larger output: 8 MB in float32, so the 8 outputs stay under 64 MB in all
+DUMP_SEED = 0
+
+
+def dump_outputs(out_dir: Path, outputs: dict) -> None:
+    """Write each output as ``out_dir/<name>.npy``: float64 arrays as they are, tensors in float32 (bf16 widened).  A tensor of
+    more than DUMP_SAMPLE elements is flattened and sampled at DUMP_SEED-seeded positions (sorted, drawn with replacement),
+    which depend only on its size: the same arguments give the same sample in every run and in every build.  None: skipped."""
+    out_dir.mkdir(parents=True, exist_ok=True)
+    total = 0
+    for name, t in outputs.items():
+        if t is None:
+            continue
+        if isinstance(t, torch.Tensor):
+            flat = t.detach().reshape(-1)
+            if flat.numel() > DUMP_SAMPLE:
+                idx = np.sort(np.random.default_rng(DUMP_SEED).integers(0, flat.numel(), DUMP_SAMPLE))
+                flat = flat[torch.from_numpy(idx).to(flat.device)]
+            t = flat.float().cpu().numpy()
+        assert t.dtype in (np.float32, np.float64), (name, t.dtype)
+        total += t.nbytes
+        assert total <= 64 << 20, f"outputs past {name} exceed 64 MB"
+        np.save(out_dir / f"{name}.npy", t)
+    log(f"dumped {', '.join(k for k, v in outputs.items() if v is not None)} ({total / 2**20:.1f} MB) to {out_dir}")
+
+
+# --------------------------------------------------------------------------------------------------
 def main() -> None:
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -219,7 +250,12 @@ def main() -> None:
     ap.add_argument("--optimizer-impl", default="fused", choices=["fused", "torch"], help="AdamW step: hand-written norm+clip+AdamW+cast+reset passes, or clip_grad_norm_ + torch.optim.AdamW(fused) + copy")
     ap.add_argument("--timeline", default="", help="write the kernel timeline of one update step per rank (CUPTI through torch.profiler, after the timed region) to <prefix>_rank<r>.json; tools/timeline_summary.py reads it")
     ap.add_argument("--dense", action="store_true", help="disable the exact token compaction (every response token through every kernel)")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR", help="after the timed update steps, write what the last one computed to DIR/<name>.npy (rank 0; see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs dumps the GPU update step; the reference arm has none")
 
     from rllm_b200.synth import WORKLOADS, make_episodes
 
@@ -251,7 +287,7 @@ def main() -> None:
             cpu_reference_step(episodes, spec, loss_kw, 64)
         vals = [cpu_reference_step(episodes, spec, loss_kw, args.cpu_sample_tokens, seed=i) for i in range(args.steps)]
         v = float(np.median([x["tokens_per_s"] for x in vals]))
-        src = "the reference's own code (unmodified install under baseline/_ref or /root/reference, third-party imports stubbed)" if vals[0]["kind"] == "reference" else "the oracle port of the reference's code"
+        src = "the reference's own code (unmodified, third-party imports stubbed)" if vals[0]["kind"] == "reference" else "the oracle port of the reference's code"
         sample = f"per step: transform + rejection filter + numpy advantages + Python prefix-merge packing + padded tensors + advantage broadcast by {src} on all {vals[0]['host_tokens']} response tokens ({vals[0]['host_s']*1e3:.0f} ms); lm_head + verl loss fwd/bwd restated in torch CPU (fp32 GEMM, all cores; the reference has no local loss) on the first {vals[0]['loss_tokens']} tokens ({vals[0]['loss_s']:.1f} s), per-token rates combined"
         emit({
             "impl": "reference", "metric": METRIC, "value": v, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup,
@@ -315,12 +351,16 @@ def main() -> None:
         pe.append((name, 0, ea, eb))
         return r
 
+    last_step = {}  # what the last device step returned beyond the metric sums (kept for --dump-outputs only)
+
     def device_step():
         phase("advantages+weights", lambda: (eng.advantages(pb, db, groups), eng.loss_weights(db)))
-        eng.forward_backward(pb, db, hidden)
+        res = eng.forward_backward(pb, db, hidden)
         phase("grad_allreduce_exposed", eng.reduce_gradients)  # the part of the all-reduce not hidden under the last dH GEMM
         sums = phase("metric_sums", eng.reduce_metrics)
-        phase("optimizer", eng.optimizer_step)
+        grad_norm = phase("optimizer", eng.optimizer_step)
+        if args.dump_outputs:
+            last_step.update(res=res, grad_norm=grad_norm)
         return sums
 
     def e2e_step():
@@ -374,6 +414,14 @@ def main() -> None:
     if rank == 0:
         sampler.start()
     dev_ms, _, sums, events = timed(device_step, args.steps, profile=True)
+    if args.dump_outputs and rank == 0:
+        res = last_step["res"]
+        master = eng._master if eng._master is not None and eng._master.shape == policy.weight.shape else None  # None: sharded (ZeRO-1)
+        dump_outputs(Path(args.dump_outputs), {
+            "advantages": db.row_adv, "logp": res.logp, "entropy": res.entropy, "d_hidden": res.d_hidden,
+            "metric_sums": np.array([sums[k] for k in L.N.SUM_NAMES], dtype=np.float64), "grad_norm": np.array([last_step["grad_norm"]], dtype=np.float64),
+            "lm_head_weight": policy.weight, "lm_head_master": master,
+        })
     launches_per_step = eng.timings.launches / args.steps + 3  # + the three advantage kernels
     for _ in range(max(1, args.warmup // 2)):
         e2e_step()
@@ -530,7 +578,7 @@ def main() -> None:
         cpu = cpu_reference_step(episodes, spec, loss_kw, args.cpu_sample_tokens)
         cpu_baseline = {
             "value": cpu["tokens_per_s"], "unit": UNIT, "cores": cores, "kind": cpu["kind"],
-            "sample": f"{'the reference itself (baseline/_ref)' if cpu['kind'] == 'reference' else 'oracle port of the reference'}: transform + filter + advantages + Python prefix-merge packing + padded tensors on all {cpu['host_tokens']} tokens ({cpu['host_s']*1e3:.0f} ms); lm_head + verl loss fwd/bwd restated in torch-CPU on {cpu['loss_tokens']} tokens ({cpu['loss_s']:.1f} s), per-token rates combined",
+            "sample": f"{'the reference itself' if cpu['kind'] == 'reference' else 'oracle port of the reference'}: transform + filter + advantages + Python prefix-merge packing + padded tensors on all {cpu['host_tokens']} tokens ({cpu['host_s']*1e3:.0f} ms); lm_head + verl loss fwd/bwd restated in torch-CPU on {cpu['loss_tokens']} tokens ({cpu['loss_s']:.1f} s), per-token rates combined",
         }
 
     if rank == 0 and args.impl == "torch_gpu" and gpu_baseline is None:

@@ -70,5 +70,5 @@ def test_reference_arm_prints_exactly_one_json_line():
         assert key in d, key
     from oracle import ref_harness
 
-    # "reference": the host stages ran on the reference's own code (/root/reference or the install under baseline/_ref); "port": oracle port
+    # "reference": the host stages ran on the reference's own code (oracle.ref_harness found a copy of it); "port": oracle port
     assert d["impl"] == "reference" and d["cpu_baseline"]["kind"] == ("reference" if ref_harness.available() else "port") and d["e2e"]["h2d_bytes_per_step"] == 0 and d["value"] > 0
