@@ -31,7 +31,7 @@
 extern "C" {
 #endif
 
-#define RLLM_B200_ABI_VERSION 2
+#define RLLM_B200_ABI_VERSION 3
 
 /* ---- library ---------------------------------------------------------------------------- */
 
@@ -103,6 +103,33 @@ int rllm_b200_pack_prefix_merge(
     int64_t* cu_resp, int32_t* resp_tok, uint8_t* resp_mask, float* resp_lp, float* resp_adv,
     uint8_t* row_has_lp,
     int64_t* out_rows, int64_t* out_tokens);
+
+/* ---- tied embeddings: fold order of the input-embedding gradient (host, C++) ------------- */
+/*
+ * In a tied model (Qwen2.5-0.5B/1.5B/3B, Llama-3.2-1B/3B) the lm_head matrix W [V, H] is also the input embedding, and
+ * its gradient is dW_lmhead + sum_p onehot(id_p) (x) d_input_embeds_p.  The reference gets the second term from autograd
+ * of the shared `embed_tokens` / `lm_head` parameter inside verl's actor update (HF / FSDP).  This builds the order in
+ * which rllm_b200_embedding_grad_accumulate adds it: a stable counting sort of the input ids, O(n + vocab).
+ *   ids        [n]       input-id stream of the shard (each row: prompt tokens, then response-region tokens)
+ * Output (caller-allocated; P = RLLM_B200_SEGMENT_PIECE):
+ *   perm       [n]             input positions sorted by id, ascending positions within an id
+ *   seg_id     [n]             id of each segment (run of equal ids in perm), ascending; n_seg used
+ *   seg_off    [n+1]           segment s = perm[seg_off[s] : seg_off[s+1]]
+ *   piece_off  [n + n/P + 1]   every segment split into pieces of at most P positions, in order:
+ *                              piece p = perm[piece_off[p] : piece_off[p+1]]
+ *   piece_row  [n + n/P]       the id (row of W) of each piece
+ *   piece_slot [n + n/P]       -1: the piece is its whole segment (adds straight into the row); else its partial's slot
+ *   multi_row  [n/P + 1]       segments of more than one piece: id
+ *   multi_slot_off [n/P + 2]   their partials: slots multi_slot_off[m] .. multi_slot_off[m+1]-1, in piece order
+ *   counts     [4]             n_seg, n_pieces, n_multi, n_slots (n_slots <= 2n/P)
+ * Ids outside [0, vocab) are an error.  n < 2^31.
+ */
+#define RLLM_B200_SEGMENT_PIECE 64
+int rllm_b200_token_segments(
+    const int32_t* ids, int64_t n, int32_t vocab,
+    int32_t* perm, int32_t* seg_id, int32_t* seg_off,
+    int32_t* piece_off, int32_t* piece_row, int32_t* piece_slot,
+    int32_t* multi_row, int32_t* multi_slot_off, int64_t* counts);
 
 /* ---- A5/A6/A7: segmented group-relative advantage (device) ------------------------------ */
 /*
@@ -430,6 +457,25 @@ int rllm_b200_adamw_step_sharded(
     float* master_dev, float* grad_dev, float* exp_avg_dev, float* exp_avg_sq_dev, void* weight_bf16_dev, int64_t n,
     float lr, float beta1, float beta2, float eps, float weight_decay, int32_t step, float max_grad_norm,
     float grad_prescale, int32_t zero_grad, const double* global_sumsq_dev, double* gnorm_dev, void* stream);
+
+/* ---- tied embeddings: the input-embedding term of the gradient (device) ------------------ */
+/*
+ * d_weight[id] += sum over the positions p with ids[p] = id, in ascending p, of d_embeds[p]   (fp32 accumulation)
+ * i.e. the embedding half of the autograd of a shared `embed_tokens` / `lm_head` parameter, which the reference runs
+ * inside verl's actor update (HF / FSDP: one parameter, two uses).  The tables are rllm_b200_token_segments' output.
+ * Pass 1: one warp per (piece, 256-column tile) sums its positions in order in fp32 registers (16-byte loads) and adds
+ * the sum to the row (a piece that is its whole segment) or writes it to partials_dev[slot]; pass 2: one warp per
+ * (multi-piece segment, tile) adds its partials in piece order and adds the sum to the row.  No atomics: every row has
+ * one writer, the result is bit-identical run to run and independent of how many SMs are free.
+ *   d_embeds_dev  bf16 [n_in, ld_in]       partials_dev  fp32 [n_slots, hidden] scratch (NULL when n_multi = 0)
+ *   d_weight_dev  fp32 [vocab, lddw]       hidden % 8 == 0, ld_in % 8 == 0, lddw % 4 == 0, 16-byte aligned rows
+ * HBM-bound: n_in * hidden * 2 + n_distinct * hidden * 8 bytes, plus 8 bytes per partial element.
+ */
+int rllm_b200_embedding_grad_accumulate(
+    const void* d_embeds_dev, int64_t ld_in, const int32_t* perm_dev,
+    const int32_t* piece_off_dev, const int32_t* piece_row_dev, const int32_t* piece_slot_dev, int32_t n_pieces,
+    const int32_t* multi_row_dev, const int32_t* multi_slot_off_dev, int32_t n_multi, float* partials_dev,
+    float* d_weight_dev, int64_t lddw, int32_t hidden, int32_t vocab, void* stream);
 
 /*
  * Test support (no reference counterpart): holds n_sms SMs for `ns` nanoseconds on `stream` (one CTA per SM that asks

@@ -14,7 +14,8 @@ _PKG_DIR = Path(__file__).resolve().parent
 LIB_PATH = _PKG_DIR / "lib" / "librllm_b200.so"
 HEADER_PATH = _PKG_DIR.parent / "include" / "rllm_b200.h"
 
-ABI_VERSION = 2
+ABI_VERSION = 3
+SEGMENT_PIECE = 64  # RLLM_B200_SEGMENT_PIECE: most input positions one warp of the tied-embedding fold sums
 
 # estimator / mode ids (keep in sync with include/rllm_b200.h)
 EST_GRPO, EST_REINFORCE, EST_RPP_BASELINE, EST_RLOO = 0, 1, 2, 3
@@ -71,6 +72,8 @@ SIGNATURES: dict[str, tuple] = {
         C.c_int,
         [_I32, _P, _P, _P, _P, _P, _P, _P, _P, _I32, _I64, _I64, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P],
     ),
+    "rllm_b200_token_segments": (C.c_int, [_P, _I64, _I32, _P, _P, _P, _P, _P, _P, _P, _P, _P]),
+    "rllm_b200_embedding_grad_accumulate": (C.c_int, [_P, _I64, _P, _P, _P, _P, _I32, _P, _P, _I32, _P, _P, _I64, _I32, _I32, _P]),
     "rllm_b200_group_advantage": (C.c_int, [_P, _P, _P, _P, _I32, _I32, _I32, _F64, _P, _P, _P, _P]),
     "rllm_b200_row_mask_counts": (C.c_int, [_P, _P, _P, _I32, _P, _P, _P]),
     "rllm_b200_row_loss_coef": (C.c_int, [_P, _I32, _I32, _F64, _F64, _F64, _P, _P]),

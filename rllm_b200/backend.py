@@ -34,12 +34,19 @@ from rllm_b200 import loss as L
 from rllm_b200.advantage import collect_reward_and_advantage_from_trajectory_groups, speculative_device_advantages
 from rllm_b200.config import SPLIT_SWEEP_LOSS_MODES, compute_schedule_lr_multiplier, AlgorithmConfig, CompactFilteringConfig, PolicyLossConfig, RejectionSamplingConfig, TransformConfig, _get
 from rllm_b200.dp import DPContext, imbalance, partition_rows
-from rllm_b200.packing import PackedBatch, pack_episodes, pack_trajectory_groups
+from rllm_b200.packing import PackedBatch, pack_episodes, pack_trajectory_groups, token_segments
 from rllm_b200.protocol import BackendProtocol
 
 
 class PolicyHead(Protocol):
-    """What the update path needs from the policy: final hidden states of the loss slots and the lm_head."""
+    """What the update path needs from the policy: final hidden states of the loss slots and the lm_head.
+
+    A head may declare ``tied_embeddings = True`` (read with ``getattr(policy, "tied_embeddings", False)``): its ``weight`` is
+    also the body's input embedding.  Its ``backward_hidden`` then returns ``d_input_embeds``, bf16 [N_in, H] on the device,
+    whose rows follow the shard's input stream (``PackedBatch.input_stream`` over the shard's rows: each row's prompt tokens,
+    then its response-region tokens), or None (nothing to fold).  The engine folds it into the lm_head gradient, so the
+    body must leave the tied matrix out of its own optimizer and take the embedding gradient through ``inputs_embeds``
+    (``F.embedding(ids, weight.detach()).requires_grad_()``), not through ``weight.grad``."""
 
     weight: torch.Tensor  # [V, H] bf16 CUDA (lm_head / tied embedding)
 
@@ -47,8 +54,9 @@ class PolicyHead(Protocol):
         """bf16 [db.n_tokens, H]: hidden state at the position *predicting* each response-region token."""
         ...
 
-    def backward_hidden(self, d_hidden: torch.Tensor) -> None:
-        """Receives d loss / d hidden (continue back-propagation into the body); may be a no-op."""
+    def backward_hidden(self, d_hidden: torch.Tensor) -> torch.Tensor | None:
+        """Receives d loss / d hidden (continue back-propagation into the body); may be a no-op.  Tied heads return
+        d loss / d input embeddings (see above)."""
         ...
 
 
@@ -73,9 +81,57 @@ class SyntheticPolicyHead:
         return None
 
 
+class SyntheticTiedPolicyHead:
+    """Tied twin of ``SyntheticPolicyHead`` (bench / tests): ``weight`` is lm_head and input embedding at once, and the body is
+    a small causal, differentiable map of the input embeddings e = weight[ids] of the shard's input stream:
+    h_p = bf16(e_p + 0.5 e_{p-1}) (e_{-1} = 0 at a row's start), read at the positions predicting the response-region tokens
+    (prompt_len - 1 + j).  ``backward_hidden`` returns the exact d loss / d e of that map (bf16 [N_in, H])."""
+
+    tied_embeddings = True
+
+    def __init__(self, vocab: int, hidden: int, device: torch.device, seed: int = 0, w_std: float = 0.02):
+        g = torch.Generator(device=device).manual_seed(seed)
+        self.vocab, self.hidden, self.device = vocab, hidden, device
+        self.weight = (torch.randn(vocab, hidden, generator=g, device=device, dtype=torch.float32) * w_std).to(torch.bfloat16)
+        self._layout: tuple | None = None  # (predicting positions, their predecessors, predecessor in the row, N_in) of the last forward
+
+    @staticmethod
+    def layout(pb: PackedBatch, rows: np.ndarray | None) -> tuple[np.ndarray, np.ndarray, np.ndarray, np.ndarray]:
+        """Input ids of the shard and, per response-region token, its predicting input position and whether that position
+        has a predecessor in its row."""
+        rows = np.arange(pb.n_rows) if rows is None else np.asarray(rows)
+        ids, cu = pb.input_stream(rows)
+        pl, rl = pb.prompt_len[rows], pb.resp_len[rows]
+        if np.any((pl == 0) & (rl > 0)):
+            raise ValueError("a row with response tokens and no prompt has no position predicting its first token")
+        within = np.arange(int(rl.sum()), dtype=np.int64) - np.repeat(np.cumsum(rl) - rl, rl)
+        q = np.repeat(cu[:-1] + pl - 1, rl) + within
+        return ids, q, q > np.repeat(cu[:-1], rl), cu
+
+    def hidden_states(self, pb: PackedBatch, db: L.DeviceBatch) -> torch.Tensor:
+        ids, q, has_prev, _ = self.layout(pb, getattr(db, "rows_global", None))
+        q_d = torch.from_numpy(q).to(self.device)
+        ok = torch.from_numpy(has_prev).to(self.device)
+        qp = torch.where(ok, q_d - 1, q_d)
+        ids_d = torch.from_numpy(ids.astype(np.int64)).to(self.device)
+        e = self.weight.index_select(0, ids_d[q_d]).float()
+        e_prev = self.weight.index_select(0, ids_d[qp]).float() * ok[:, None]
+        self._layout = (q_d, qp[ok], ok, len(ids))
+        return (e + 0.5 * e_prev).to(torch.bfloat16)
+
+    def backward_hidden(self, d_hidden: torch.Tensor) -> torch.Tensor:
+        q, qp, ok, n_in = self._layout
+        g = d_hidden.float()
+        d_in = torch.zeros(n_in, self.hidden, dtype=torch.float32, device=self.device)
+        d_in.index_copy_(0, q, g)  # predicting positions are distinct, and so are their predecessors: no two writers
+        d_in.index_add_(0, qp, 0.5 * g[ok])
+        return d_in.to(torch.bfloat16)
+
+
 @dataclass
 class UpdateTimings:
     pack_s: float = 0.0
+    segment_s: float = 0.0  # tied heads: host build of the input-embedding fold order (input stream + counting sort)
     h2d_bytes: int = 0
     d2h_bytes: int = 0
     launches: int = 0
@@ -307,6 +363,12 @@ class PolicyUpdateEngine:
             pb.meta_info["dp"] = {k: v for k, v in pb.meta_info["shard"].items() if k.startswith("dp/")}
         db = L.DeviceBatch.from_packed(pb, self.device, rows)
         db.rows_global = rows  # type: ignore[attr-defined]
+        if self.tied:  # the input ids are host data here: build the fold order of the embedding gradient now, upload it with the shard
+            t0 = time.perf_counter()
+            ids, _ = pb.input_stream(self._shard_rows(pb, db))
+            seg = token_segments(ids, self.policy.weight.shape[0])
+            self.timings.segment_s = time.perf_counter() - t0
+            db.embed_segments = L.DeviceSegments.from_host(seg, self.device)
         self.timings.h2d_bytes = db.h2d_bytes()
         return db
 
@@ -321,6 +383,8 @@ class PolicyUpdateEngine:
         groups' rewards and the algorithm config, so they are computed here on the device WITHOUT touching any Step
         (``speculative_device_advantages``); stage 6 still does the mutation / metrics, and a plan that turns out different
         (custom estimator, changed config) simply makes the update recompute its forward."""
+        if self.tied:
+            self.wait_weights()  # a tied body reads policy.weight for its embedding lookup
         hidden = self.policy.hidden_states(pb, db) if hidden is None else hidden
         self.wait_weights()
         self._resident = None
@@ -423,6 +487,9 @@ class PolicyUpdateEngine:
         return n_tok, n_seq
 
     def forward_backward(self, pb: PackedBatch, db: L.DeviceBatch, hidden: torch.Tensor | None = None, cfg: PolicyLossConfig | None = None, row_select: np.ndarray | None = None) -> L.HeadLossResult:
+        tied = self.tied
+        if tied:
+            self.wait_weights()  # a tied body reads policy.weight for its embedding lookup
         hidden = self.policy.hidden_states(pb, db) if hidden is None else hidden
         self.wait_weights()
         cfg = cfg or self.loss_config
@@ -430,7 +497,9 @@ class PolicyUpdateEngine:
         if self.d_weight is None:
             self.d_weight = torch.zeros(V, H, dtype=torch.float32, device=self.device)
         self._grad_handle = None
-        overlap = self.dp.enabled and self.overlap_grad_allreduce and self.accum_passes == 0 and not getattr(self, "_accumulating", False)
+        # tied: the embedding term is folded in after the sweep, so no slice is final inside it; reduce_gradients exchanges
+        # the whole gradient afterwards
+        overlap = self.dp.enabled and self.overlap_grad_allreduce and self.accum_passes == 0 and not getattr(self, "_accumulating", False) and not tied
         handles: list = []
         self.head.grad_slices = self.grad_allreduce_slices if overlap else 1
         self.head.on_dweight_final = (lambda g: (handles.append(self._reduce_slice_async(g)), setattr(self, "_grad_handle", handles))) if overlap else None
@@ -447,9 +516,23 @@ class PolicyUpdateEngine:
         else:
             res = self.head.forward_backward(hidden, self.policy.weight, db, cfg, d_weight=self.d_weight)
         self._take_probe()
-        self.policy.backward_hidden(res.d_hidden)
+        d_in = self.policy.backward_hidden(res.d_hidden)
+        if tied and d_in is not None:
+            self._fold_embedding_grad(db, d_in)
         self.timings.launches += res.launches
         return res
+
+    @property
+    def tied(self) -> bool:
+        """The head's weight is also the body's input embedding (``PolicyHead.tied_embeddings``)."""
+        return bool(getattr(self.policy, "tied_embeddings", False))
+
+    def _fold_embedding_grad(self, db: L.DeviceBatch, d_in: torch.Tensor) -> None:
+        """d_weight += the input-embedding term of a tied head's gradient (rllm_b200_embedding_grad_accumulate)."""
+        seg = db.embed_segments
+        if seg is None:
+            raise RuntimeError("tied head: the batch carries no embedding fold order (build the device batch with PolicyUpdateEngine.shard_to_device)")
+        self.timings.launches += L.embedding_grad_accumulate(d_in, seg, self.d_weight)
 
     def _take_probe(self) -> None:
         """Throughput sample of the sweep that just ran (FusedLMHeadLoss.probe: its collective-free part), for the balancer."""

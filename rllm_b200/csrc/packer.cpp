@@ -133,3 +133,51 @@ extern "C" int rllm_b200_pack_prefix_merge(int32_t n_traj, const int64_t* traj_s
   *out_tokens = cursor;
   return 0;
 }
+
+// Fold order of a tied head's input-embedding gradient (rllm_b200_embedding_grad_accumulate): stable counting sort of the
+// shard's input ids, O(n + vocab), then every run of equal ids cut into pieces of at most RLLM_B200_SEGMENT_PIECE positions so
+// that a frequent id (newline, the prompt every rollout of a group repeats) is summed by several warps, not one.
+extern "C" int rllm_b200_token_segments(const int32_t* ids, int64_t n, int32_t vocab, int32_t* perm, int32_t* seg_id, int32_t* seg_off,
+                                        int32_t* piece_off, int32_t* piece_row, int32_t* piece_slot, int32_t* multi_row, int32_t* multi_slot_off,
+                                        int64_t* counts) {
+  if (n < 0 || n > INT32_MAX - 1 || vocab <= 0 || !seg_off || !piece_off || !multi_slot_off || !counts || (n > 0 && (!ids || !perm || !seg_id || !piece_row || !piece_slot))) {
+    rb::set_error("token_segments: bad arguments (n=%lld, vocab=%d)", static_cast<long long>(n), vocab);
+    return 1;
+  }
+  constexpr int32_t P = RLLM_B200_SEGMENT_PIECE;
+  std::vector<int32_t> start(static_cast<size_t>(vocab) + 1, 0);
+  for (int64_t i = 0; i < n; ++i) {
+    const int32_t v = ids[i];
+    if (v < 0 || v >= vocab) {
+      rb::set_error("token_segments: id %d at position %lld outside [0, %d)", v, static_cast<long long>(i), vocab);
+      return 1;
+    }
+    ++start[static_cast<size_t>(v) + 1];
+  }
+  for (int32_t v = 0; v < vocab; ++v) start[v + 1] += start[v];
+  int64_t n_seg = 0, n_pieces = 0, n_multi = 0, n_slots = 0;
+  seg_off[0] = piece_off[0] = multi_slot_off[0] = 0;
+  for (int32_t v = 0; v < vocab; ++v) {  // segments and pieces, ascending id (positions are placed below)
+    const int32_t a = start[v], b = start[v + 1];
+    if (a == b) continue;
+    seg_id[n_seg] = v;
+    seg_off[++n_seg] = b;
+    const int32_t k = (b - a + P - 1) / P;
+    for (int32_t j = 0; j < k; ++j) {
+      piece_row[n_pieces] = v;
+      piece_slot[n_pieces] = k == 1 ? -1 : static_cast<int32_t>(n_slots + j);
+      piece_off[++n_pieces] = std::min(b, a + (j + 1) * P);
+    }
+    if (k > 1) {
+      multi_row[n_multi] = v;
+      n_slots += k;
+      multi_slot_off[++n_multi] = static_cast<int32_t>(n_slots);
+    }
+  }
+  for (int64_t i = 0; i < n; ++i) perm[start[ids[i]]++] = static_cast<int32_t>(i);  // stable: ascending positions within an id
+  counts[0] = n_seg;
+  counts[1] = n_pieces;
+  counts[2] = n_multi;
+  counts[3] = n_slots;
+  return 0;
+}

@@ -71,6 +71,7 @@ class DeviceBatch:
     tok_adv: torch.Tensor | None = None  # float32 [T] per-token advantages (pre-computed lists); replaces row_adv
     row_aux: torch.Tensor | None = None  # float32 [B] GSPO: log sequence importance ratio per row
     lse_ref: torch.Tensor | None = None  # float32 [T] log-sum-exp of every token from the pi_old pass: the per-token reference of the exponential operand
+    embed_segments: "DeviceSegments | None" = None  # tied heads only: fold order of the input-embedding gradient (packing.TokenSegments)
 
     @classmethod
     def from_packed(cls, pb, device: torch.device | None = None, rows: np.ndarray | None = None) -> "DeviceBatch":
@@ -109,7 +110,53 @@ class DeviceBatch:
         )
 
     def h2d_bytes(self) -> int:
-        return sum(t.numel() * t.element_size() for t in (self.cu_resp, self.labels, self.mask, self.rollout_logp, self.row_valid, self.row_traj))
+        seg = 0 if self.embed_segments is None else self.embed_segments.table.numel() * 4
+        return seg + sum(t.numel() * t.element_size() for t in (self.cu_resp, self.labels, self.mask, self.rollout_logp, self.row_valid, self.row_traj))
+
+
+@dataclass
+class DeviceSegments:
+    """``packing.TokenSegments`` on the device: one int32 table (one H2D) and views of its parts."""
+
+    n_in: int
+    n_pieces: int
+    n_multi: int
+    n_slots: int
+    table: torch.Tensor
+    parts: dict
+
+    @classmethod
+    def from_host(cls, seg, device: torch.device) -> "DeviceSegments":
+        t = torch.from_numpy(seg.table)
+        if t.numel():
+            t = t.pin_memory()
+        t = t.to(device, non_blocking=True)
+        parts, o = {}, 0
+        for name, n in zip(seg.FIELDS, seg.sizes()):
+            parts[name] = t[o : o + n]
+            o += n
+        return cls(seg.n_in, seg.n_pieces, seg.n_multi, seg.n_slots, t, parts)
+
+
+def embedding_grad_accumulate(d_embeds: torch.Tensor, seg: DeviceSegments, d_weight: torch.Tensor) -> int:
+    """d_weight[id] += sum of the d_embeds rows of the positions holding that id, in ascending position (the input-embedding
+    term of a tied lm_head's gradient; deterministic, no atomics).  Returns the number of kernel launches."""
+    _require_cuda(d_embeds, "d_embeds")
+    _require_cuda(d_weight, "d_weight")
+    if d_embeds.dtype != torch.bfloat16 or d_embeds.dim() != 2 or d_embeds.stride(1) != 1 or d_embeds.shape[0] != seg.n_in:
+        raise ValueError(f"d_embeds must be a row-major bf16 [{seg.n_in}, H] tensor, got {tuple(d_embeds.shape)} {d_embeds.dtype}")
+    if d_weight.dtype != torch.float32 or d_weight.stride(1) != 1 or d_weight.shape[1] != d_embeds.shape[1]:
+        raise ValueError("d_weight must be a row-major fp32 [V, H] tensor with the same H as d_embeds")
+    if seg.n_pieces == 0:
+        return 0
+    V, H = d_weight.shape
+    partials = torch.empty(seg.n_slots, H, dtype=torch.float32, device=d_weight.device) if seg.n_multi else None
+    p = seg.parts
+    N.check(N.lib().rllm_b200_embedding_grad_accumulate(
+        N.ptr(d_embeds), d_embeds.stride(0), N.ptr(p["perm"]), N.ptr(p["piece_off"]), N.ptr(p["piece_row"]), N.ptr(p["piece_slot"]), seg.n_pieces,
+        N.ptr(p["multi_row"]), N.ptr(p["multi_slot_off"]), seg.n_multi, N.ptr(partials), N.ptr(d_weight), d_weight.stride(0), H, V, N.current_stream_ptr()),
+        "rllm_b200_embedding_grad_accumulate")
+    return 2 if seg.n_multi else 1
 
 
 def row_mask_counts(db: DeviceBatch) -> None:
